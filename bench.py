@@ -2,7 +2,7 @@
 """bench.py -- the reference's headline benchmark (BASELINE.json configs[1]): gemm_i4_o16, M=16, N=K=4096,
 group 128, INT8 keeper 128, on synthetic random-quantised operands.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--m M]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--m M] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Besides the headline line this also reports, in the same JSON object:
@@ -19,6 +19,11 @@ reference's convention, bench_dense_layer_gemm_i4_o16.cu:40-42); multi-GPU runs 
 scaling, no data-path collective: GEMM problems are independent units).  `e2e` = the same metric through the public
 operator (atom_b200.ops.dense_layer_gemm_i4_fp16) with HOST activations: per step one pinned H2D copy of the quantised
 activation tuple, the GEMM, and a D2H read of the FP16 result.
+
+--dump-outputs DIR writes, after the timed steps, what the last step returned to its caller as float32 .npy files (rank 0):
+gemm_out.npy is the [M, N] result of the last GEMM of the last headline step (every GEMM of a step computes on a copy of the
+same operands), e2e_out.npy the host result of the last e2e step.  The operands come from fixed seeds, so two builds run with
+the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -28,12 +33,14 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
 L2_BYTES = 126e6
+DUMP_BYTES = 60 << 20          # --dump-outputs: under 64 MB in all, .npy headers included
 
 # BASELINE.md section 1: the reference's published bench_gemm_i4_o16 numbers (RTX 4090, figures/bench_gemm.png), TOP/s by M
 PUBLISHED_TOPS = {16: 20.079, 32: 38.334, 64: 78.997, 128: 151.281, 256: 312.242, 512: 546.035, 1024: 630.779,
@@ -103,6 +110,20 @@ def cpu_baseline(m, n, k, budget_s=12.0):
     tops = 2.0 * m * n * k * it / el * 1e-12
     return {"value": tops, "unit": "TOP/s", "cores": cores, "kind": "port",
             "sample": f"{it} forwards of the fake-quant W4A4 linear (fp32 torch, act quant + F.linear) at M={m}, N={n}, K={k} in {el:.1f} s"}
+
+
+def dump_outputs(dirname, arrays):
+    """Writes each array as DIRNAME/<name>.npy in float32.  Above DUMP_BYTES in all, every array keeps the same share of
+    its elements, drawn with a fixed seed (flattened, in index order), so that runs stay comparable element for element."""
+    os.makedirs(dirname, exist_ok=True)
+    total = sum(a.numel() for a in arrays.values()) * 4
+    for name, a in arrays.items():
+        a = a.detach().float()
+        if total > DUMP_BYTES:
+            keep = a.numel() * DUMP_BYTES // total
+            idx = np.unique(np.random.default_rng(0).integers(0, a.numel(), keep))
+            a = a.reshape(-1)[torch.from_numpy(idx).to(a.device)]
+        np.save(os.path.join(dirname, name + ".npy"), a.cpu().numpy())
 
 
 def ncu_traffic(m):
@@ -251,6 +272,7 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-sweep", action="store_true")
     ap.add_argument("--no-tp", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy (float32)")
     a = ap.parse_args()
     M, N, K = a.m, 4096, 4096
     rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
@@ -296,22 +318,25 @@ def main():
     stream = torch.cuda.default_stream(dev) if ref_mode else torch.cuda.Stream(dev)
 
     def run_batch():
+        """Runs one step's GEMMs and returns the result of the last one."""
         if ref_mode:   # the reference launches on the legacy default stream (GEMM.cuh:763): not capturable, plain loop
             for i in range(R_sets):
                 R.gemm_i4_o16(*sets[i], d=outs[i], sync=0)
-        else:
-            for i in range(R_sets):
-                ops.dense_layer_gemm_i4_fp16(*sets[i])
+            return outs[-1]
+        # results are dropped as they come, so the allocator can hand one output buffer to every GEMM of the step
+        for i in range(R_sets - 1):
+            ops.dense_layer_gemm_i4_fp16(*sets[i])
+        return ops.dense_layer_gemm_i4_fp16(*sets[-1])
 
     graph = None
     with torch.cuda.stream(stream):
-        run_batch()
+        last_out = run_batch()
         stream.synchronize()
         torch.cuda.synchronize()
         if not ref_mode:
             graph = torch.cuda.CUDAGraph()
             with torch.cuda.graph(graph, stream=stream):
-                run_batch()
+                last_out = run_batch()        # every replay rewrites this tensor
 
     launch_desc = "one CUDA graph replay per step" if graph is not None else "python loop on the legacy stream (reference launcher)"
 
@@ -351,6 +376,7 @@ def main():
         # of the host's wall clock between the two synchronising barriers; a large gap means they did not bracket the work
         assert ms >= 0.7 * wall_ms - 1.0, f"timing contract broken: events {ms:.3f} ms vs wall clock {wall_ms:.3f} ms"
     clocks = sampler.stop() if rank == 0 else None
+    dumped = {"gemm_out": last_out.clone()} if a.dump_outputs and rank == 0 else None
     t = torch.tensor([ms], device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -419,6 +445,9 @@ def main():
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     e2e_tops = op_count * e2e_steps * world / t.item() * 1e-12
+    if dumped is not None:
+        dumped["e2e_out"] = host_out.clone()
+        dump_outputs(a.dump_outputs, dumped)
     # self-check of the timing contract: one device-timed launch cannot take longer than a whole synchronised e2e step
     # (H2D + the same launch + D2H + sync); if it does, the events did not bracket the kernels
     e2e_us_per_step = t.item() / e2e_steps * 1e6
