@@ -20,7 +20,6 @@
 #include "gemm_i4_sm100.cuh"
 #include "gemm_i4_skinny_sm100.cuh"
 #include "gemm_i4_tall_sm100.cuh"
-#include "gemm_i4_wide_sm100.cuh"
 #include "kv_kernels.cuh"
 #include "prefill_kernels.cuh"
 #include "comm_kernels.cuh"
@@ -63,24 +62,39 @@ int check_launch(const char* what) {
   return ATOM_OK;
 }
 
-// <<<>>> when PDL is off (the validated path, untouched); cudaLaunchKernelEx with the attribute when it is on
+// Every kernel of the library except the prefill-attention and stand-alone all-reduce kernels is launched here:
+// cluster_z > 0 adds a (1, 1, cluster_z) thread-block cluster, pdl programmatic stream serialization.
+template <typename... KArgs, typename... Args>
+int launch(const char* what, void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, int cluster_z,
+           bool pdl, Args... args) {
+  cudaLaunchConfig_t cfg{};
+  cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = stream;
+  cudaLaunchAttribute attr[2];
+  unsigned n = 0;
+  if (cluster_z > 0) {
+    attr[n].id = cudaLaunchAttributeClusterDimension;
+    attr[n].val.clusterDim.x = 1; attr[n].val.clusterDim.y = 1; attr[n].val.clusterDim.z = (unsigned)cluster_z;
+    ++n;
+  }
+  if (pdl) {
+    attr[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[n].val.programmaticStreamSerializationAllowed = 1;
+    ++n;
+  }
+  cfg.attrs = attr; cfg.numAttrs = n;
+  cudaError_t e = cudaLaunchKernelEx(&cfg, kern, args...);
+  if (e != cudaSuccess) {
+    (void)cudaGetLastError();   // the failure is reported here; do not leave it for the caller's next launch check
+    return fail(ATOM_E_CUDA, "%s launch: %s", what, cudaGetErrorString(e));
+  }
+  return ATOM_OK;
+}
+
+// The non-GEMM kernels take a trailing `pdl` argument and follow pdl_enabled().
 template <typename... KArgs, typename... Args>
 int launch_k(const char* what, void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, Args... args) {
-  if (!pdl_enabled()) {
-    kern<<<grid, block, smem, stream>>>(args..., 0);
-  } else {
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr; cfg.numAttrs = 1;
-    cudaError_t e = cudaLaunchKernelEx(&cfg, kern, args..., 1);
-    if (e != cudaSuccess) return fail(ATOM_E_CUDA, "%s launch: %s", what, cudaGetErrorString(e));
-  }
-  cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) return fail(ATOM_E_CUDA, "%s: %s", what, cudaGetErrorString(e));
-  return ATOM_OK;
+  const bool pdl = pdl_enabled();
+  return launch(what, kern, grid, block, smem, stream, 0, pdl, args..., pdl ? 1 : 0);
 }
 
 inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
@@ -122,29 +136,36 @@ EncodeFn encode_fn() {
   return fn;
 }
 
+// Everything that determines a descriptor; unused trailing dimensions stay zero.  No padding: compared bytewise.
 struct MapKey {
-  const void* ptr; uint64_t inner, rows, pitch; uint32_t box_inner, box_rows, swizzle;
-  bool operator==(const MapKey& o) const {
-    return ptr == o.ptr && inner == o.inner && rows == o.rows && pitch == o.pitch && box_inner == o.box_inner &&
-           box_rows == o.box_rows && swizzle == o.swizzle;
-  }
+  const void* ptr; uint32_t rank, swizzle; cuuint64_t dims[4], strides[3]; cuuint32_t box[4];
+  bool operator==(const MapKey& o) const { return memcmp(this, &o, sizeof(MapKey)) == 0; }
 };
+static_assert(sizeof(MapKey) == 8 + 2 * 4 + 7 * 8 + 4 * 4, "MapKey must have no padding bytes");
 struct MapKeyHash {
   size_t operator()(const MapKey& k) const {
     size_t h = reinterpret_cast<size_t>(k.ptr);
     auto mix = [&](uint64_t v) { h ^= v + 0x9e3779b97f4a7c15ull + (h << 6) + (h >> 2); };
-    mix(k.inner); mix(k.rows); mix(k.pitch); mix(k.box_inner); mix(k.box_rows); mix(k.swizzle);
+    mix(k.rank); mix(k.swizzle);
+    for (cuuint64_t d : k.dims) mix(d);
+    for (cuuint64_t s : k.strides) mix(s);
+    for (cuuint32_t b : k.box) mix(b);
     return h;
   }
 };
 std::mutex g_map_mu;
 std::unordered_map<MapKey, CUtensorMap, MapKeyHash> g_maps;
 
-// 2-D byte tensor [rows][inner] with row pitch `pitch`; box = box_rows x box_inner bytes; OOB rows read as zero.
-// swizzle: 0 = none, 1 = SWIZZLE_128B, 2 = SWIZZLE_64B
-int make_map(CUtensorMap* out, const void* ptr, uint64_t inner, uint64_t rows, uint64_t pitch, uint32_t box_inner,
-             uint32_t box_rows, int swizzle) {
-  MapKey key{ptr, inner, rows, pitch, box_inner, box_rows, (uint32_t)swizzle};
+// Byte tensor of `rank` <= 4 dimensions (dims[0] contiguous, strides[i] = pitch of dimension i+1 in bytes), box in
+// elements per dimension; elements outside the tensor read as zero.  swizzle: 0 = none, 1 = SWIZZLE_128B, 2 = SWIZZLE_64B.
+// Descriptors are cached by everything that determines them (the cache is dropped once it exceeds 4096 entries).
+int encode_map(CUtensorMap* out, const void* ptr, uint32_t rank, const cuuint64_t* dims, const cuuint64_t* strides,
+               const cuuint32_t* box, int swizzle) {
+  MapKey key{};
+  key.ptr = ptr; key.rank = rank; key.swizzle = (uint32_t)swizzle;
+  std::copy(dims, dims + rank, key.dims);
+  std::copy(strides, strides + rank - 1, key.strides);
+  std::copy(box, box + rank, key.box);
   {
     std::lock_guard<std::mutex> lk(g_map_mu);
     auto it = g_maps.find(key);
@@ -152,19 +173,24 @@ int make_map(CUtensorMap* out, const void* ptr, uint64_t inner, uint64_t rows, u
   }
   EncodeFn fn = encode_fn();
   if (!fn) return fail(ATOM_E_CUDA, "cuTensorMapEncodeTiled is not available from this driver");
-  cuuint64_t dims[2] = {inner, rows};
-  cuuint64_t strides[1] = {pitch};
-  cuuint32_t box[2] = {box_inner, box_rows};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(out, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, const_cast<void*>(ptr), dims, strides, box, estr,
+  const cuuint32_t estr[4] = {1, 1, 1, 1};
+  CUresult r = fn(out, CU_TENSOR_MAP_DATA_TYPE_UINT8, rank, const_cast<void*>(ptr), key.dims, key.strides, key.box, estr,
                   CU_TENSOR_MAP_INTERLEAVE_NONE,
                   swizzle == 1 ? CU_TENSOR_MAP_SWIZZLE_128B : (swizzle == 2 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_NONE),
                   CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) return fail(ATOM_E_CUDA, "cuTensorMapEncodeTiled failed with CUresult %d", (int)r);
+  if (r != CUDA_SUCCESS) return fail(ATOM_E_CUDA, "cuTensorMapEncodeTiled (%u-D) failed with CUresult %d", rank, (int)r);
   std::lock_guard<std::mutex> lk(g_map_mu);
   if (g_maps.size() > 4096) g_maps.clear();
   g_maps.emplace(key, *out);
   return ATOM_OK;
+}
+
+// 2-D byte matrix [rows][inner] with row pitch `pitch`; box = box_rows x box_inner bytes.
+int make_map(CUtensorMap* out, const void* ptr, uint64_t inner, uint64_t rows, uint64_t pitch, uint32_t box_inner,
+             uint32_t box_rows, int swizzle) {
+  const cuuint64_t dims[2] = {inner, rows}, strides[1] = {pitch};
+  const cuuint32_t box[2] = {box_inner, box_rows};
+  return encode_map(out, ptr, 2, dims, strides, box, swizzle);
 }
 
 // The same byte matrix viewed as [rows/4][2][2][inner] with the two middle dimensions swapped: a box of `box_rows` rows
@@ -172,26 +198,9 @@ int make_map(CUtensorMap* out, const void* ptr, uint64_t inner, uint64_t rows, u
 // then belong to different channel pairs).  rows % 4 == 0; rows beyond the matrix read as zero.
 int make_map_quadswap(CUtensorMap* out, const void* ptr, uint64_t inner, uint64_t rows, uint64_t pitch, uint32_t box_inner,
                       uint32_t box_rows, int swizzle) {
-  MapKey key{ptr, inner, rows, pitch, box_inner, box_rows, (uint32_t)swizzle | 0x100u};
-  {
-    std::lock_guard<std::mutex> lk(g_map_mu);
-    auto it = g_maps.find(key);
-    if (it != g_maps.end()) { *out = it->second; return ATOM_OK; }
-  }
-  EncodeFn fn = encode_fn();
-  if (!fn) return fail(ATOM_E_CUDA, "cuTensorMapEncodeTiled is not available from this driver");
-  cuuint64_t dims[4] = {inner, 2, 2, (rows + 3) / 4};
-  cuuint64_t strides[3] = {2 * pitch, pitch, 4 * pitch};
-  cuuint32_t box[4] = {box_inner, 2, 2, box_rows / 4};
-  cuuint32_t estr[4] = {1, 1, 1, 1};
-  CUresult r = fn(out, CU_TENSOR_MAP_DATA_TYPE_UINT8, 4, const_cast<void*>(ptr), dims, strides, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle == 1 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_NONE,
-                  CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) return fail(ATOM_E_CUDA, "cuTensorMapEncodeTiled (4-D) failed with CUresult %d", (int)r);
-  std::lock_guard<std::mutex> lk(g_map_mu);
-  if (g_maps.size() > 4096) g_maps.clear();
-  g_maps.emplace(key, *out);
-  return ATOM_OK;
+  const cuuint64_t dims[4] = {inner, 2, 2, (rows + 3) / 4}, strides[3] = {2 * pitch, pitch, 4 * pitch};
+  const cuuint32_t box[4] = {box_inner, 2, 2, box_rows / 4};
+  return encode_map(out, ptr, 4, dims, strides, box, swizzle);
 }
 
 // ------------------------------------------------------------------------------------------------ GEMM launch
@@ -200,44 +209,24 @@ struct GemmOperands {
   int64_t M, N, K;
 };
 
-template <bool kSwap, int BN, int GS, int kPack, int kSplit, bool kO4, int kConvWarps, int kEpiWgs>
+// Weight-stationary kernel for 33-128 tokens (gemm_i4_sm100.cuh): always launched as a cluster of kSplit CTAs along z.
+template <int GS, int kPack, int kSplit, bool kO4>
 int launch_gemm(const GemmOperands& op, const atom::GemmArgs& args, cudaStream_t stream) {
-  using C = atom::GemmCfg<kSwap, BN, GS, kPack, kSplit, kO4, kConvWarps, kEpiWgs>;
-  auto kern = atom::gemm_i4_kernel<kSwap, BN, GS, kPack, kSplit, kO4, kConvWarps, kEpiWgs>;
+  using C = atom::GemmCfg<GS, kPack, kSplit, kO4>;
+  auto kern = atom::gemm_i4_kernel<GS, kPack, kSplit, kO4>;
   int rc = ensure_dynamic_smem(kern, C::SMEM_BYTES, "gemm_i4");
   if (rc) return rc;
   const uint64_t kp = (uint64_t)(op.K - 128) / 2;
-  // MMA-M operand = kSwap ? weights : tokens
-  const void* p4 = kSwap ? op.b : op.a;  const void* q4 = kSwap ? op.a : op.b;
-  const void* p8 = kSwap ? op.bk : op.ak; const void* q8 = kSwap ? op.ak : op.bk;
-  const uint64_t prow = kSwap ? op.N : op.M, qrow = kSwap ? op.M : op.N;
-  CUtensorMap tp4, tq4, tp8, tq8;
-  if ((rc = make_map(&tp4, p4, kp, prow, kp, 64, C::BM, 0))) return rc;
-  if ((rc = make_map(&tq4, q4, kp, qrow, kp, 64, BN, 0))) return rc;
-  if ((rc = make_map(&tp8, p8, 128, prow, 128, 128, C::BM, 1))) return rc;
-  if ((rc = make_map(&tq8, q8, 128, qrow, 128, 128, BN, 1))) return rc;
-
-  const int ch_tile = kSwap ? C::BM : BN, tok_tile = kSwap ? BN : C::BM;
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3((unsigned)((op.N + ch_tile - 1) / ch_tile), (unsigned)((op.M + tok_tile - 1) / tok_tile), kSplit);
-  cfg.blockDim = dim3(C::THREADS);
-  cfg.dynamicSmemBytes = C::SMEM_BYTES;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[2];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 1; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = kSplit;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
+  CUtensorMap tp4, tq4, tp8, tq8;   // P = weights (MMA-M), Q = tokens (MMA-N)
+  if ((rc = make_map(&tp4, op.b, kp, op.N, kp, 64, C::BM, 0))) return rc;
+  if ((rc = make_map(&tq4, op.a, kp, op.M, kp, 64, C::BN, 0))) return rc;
+  if ((rc = make_map(&tp8, op.bk, 128, op.N, 128, 128, C::BM, 1))) return rc;
+  if ((rc = make_map(&tq8, op.ak, 128, op.M, 128, 128, C::BN, 1))) return rc;
+  const dim3 grid((unsigned)((op.N + C::BM - 1) / C::BM), (unsigned)((op.M + C::BN - 1) / C::BN), kSplit);
+  const bool pdl = pdl_enabled();
   atom::GemmArgs largs = args;
-  if (pdl_enabled()) {
-    attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[1].val.programmaticStreamSerializationAllowed = 1;
-    cfg.numAttrs = 2;
-    largs.pdl = 1;
-  }
-  cudaError_t e = cudaLaunchKernelEx(&cfg, kern, tp4, tq4, tp8, tq8, largs);
-  if (e != cudaSuccess) return fail(ATOM_E_CUDA, "gemm_i4 launch: %s", cudaGetErrorString(e));
-  return ATOM_OK;
+  if (pdl) largs.pdl = 1;
+  return launch("gemm_i4", kern, grid, dim3(C::THREADS), C::SMEM_BYTES, stream, kSplit, pdl, tp4, tq4, tp8, tq8, largs);
 }
 
 // Decode-shape kernel (gemm_i4_skinny_sm100.cuh): weights expanded into tensor memory, two CTAs per SM, always launched
@@ -261,30 +250,15 @@ int launch_skinny(const GemmOperands& op, const atom::GemmArgs& args, cudaStream
   CUtensorMap tp4, tp8;       // weights only: the token operand is read with plain loads (no descriptor per activation buffer)
   if ((rc = make_map(&tp4, op.b, kp, op.N, kp, 64, C::BM, 2))) return rc;
   if ((rc = make_map(&tp8, op.bk, 128, op.N, 128, 128, C::BM, 1))) return rc;
-  cudaLaunchConfig_t cfg{};
   const int64_t chan = out_channels > 0 ? out_channels : op.N;       // (gate/up: op.N = 2 I weight rows, I output channel tiles)
-  cfg.gridDim = dim3((unsigned)((chan + C::BM - 1) / C::BM), (unsigned)((op.M + BN - 1) / BN), kSplit);
-  cfg.blockDim = dim3(C::THREADS);
-  cfg.dynamicSmemBytes = C::SMEM_BYTES;
+  const dim3 grid((unsigned)((chan + C::BM - 1) / C::BM), (unsigned)((op.M + BN - 1) / BN), kSplit);
+  size_t smem = C::SMEM_BYTES;
   if (kEpi == atom::EPI_GATEUP && (args.dbg & 2) && C::SMEM_BYTES < 120 * 1024) {     // experiment: one CTA per SM
     static bool raised = false;
     if (!raised) { cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 120 * 1024); raised = true; }
-    cfg.dynamicSmemBytes = 120 * 1024;
+    smem = 120 * 1024;
   }
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[2];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 1; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = kSplit;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  if (gemm_pdl_enabled()) {
-    attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[1].val.programmaticStreamSerializationAllowed = 1;
-    cfg.numAttrs = 2;
-  }
-  cudaError_t e = cudaLaunchKernelEx(&cfg, kern, tp4, tp8, args);
-  if (e != cudaSuccess) return fail(ATOM_E_CUDA, "gemm_i4 (skinny) launch: %s", cudaGetErrorString(e));
-  return ATOM_OK;
+  return launch("gemm_i4 (skinny)", kern, grid, dim3(C::THREADS), smem, stream, kSplit, gemm_pdl_enabled(), tp4, tp8, args);
 }
 
 // Prefill-shape kernel (gemm_i4_tall_sm100.cuh): biased accumulators, packed FP32 epilogue, TMA-permuted weight rows.
@@ -300,53 +274,8 @@ int launch_tall(const GemmOperands& op, const atom::GemmArgs& args, cudaStream_t
   if ((rc = make_map_quadswap(&tq4, op.b, kp, op.N, kp, 64, C::BN, 0))) return rc;
   if ((rc = make_map(&tp8, op.ak, 128, op.M, 128, 128, C::BM, 1))) return rc;
   if ((rc = make_map_quadswap(&tq8, op.bk, 128, op.N, 128, 128, C::BN, 1))) return rc;
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3((unsigned)((op.N + C::BN - 1) / C::BN), (unsigned)((op.M + C::BM - 1) / C::BM), 1);
-  cfg.blockDim = dim3(C::THREADS);
-  cfg.dynamicSmemBytes = C::SMEM_BYTES;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[1];
-  cfg.attrs = attr;
-  cfg.numAttrs = 0;
-  if (gemm_pdl_enabled()) {
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.numAttrs = 1;
-  }
-  cudaError_t e = cudaLaunchKernelEx(&cfg, kern, tp4, tq4, tp8, tq8, args);
-  if (e != cudaSuccess) return fail(ATOM_E_CUDA, "gemm_i4 (tall) launch: %s", cudaGetErrorString(e));
-  return ATOM_OK;
-}
-
-// Prefill-shape kernel with the token operand in tensor memory, 128 x 256 tiles (gemm_i4_wide_sm100.cuh).
-template <bool kO4>
-int launch_wide(const GemmOperands& op, const atom::GemmArgs& args, cudaStream_t stream) {
-  using C = atom::WideCfg<kO4>;
-  auto kern = atom::gemm_i4_wide_kernel<kO4>;
-  int rc = ensure_dynamic_smem(kern, C::SMEM_BYTES, "gemm_i4 (wide)");
-  if (rc) return rc;
-  const uint64_t kp = (uint64_t)(op.K - 128) / 2;
-  CUtensorMap ta4, tb4, ta8, tb8;
-  if ((rc = make_map(&ta4, op.a, kp, op.M, kp, 64, C::BM, 2))) return rc;
-  if ((rc = make_map_quadswap(&tb4, op.b, kp, op.N, kp, 64, C::BH, 0))) return rc;
-  if ((rc = make_map(&ta8, op.ak, 128, op.M, 128, 128, C::BM, 1))) return rc;
-  if ((rc = make_map_quadswap(&tb8, op.bk, 128, op.N, 128, 128, C::BH, 1))) return rc;
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3((unsigned)((op.N + C::NH * C::BH - 1) / (C::NH * C::BH)), (unsigned)((op.M + C::BM - 1) / C::BM), 1);
-  cfg.blockDim = dim3(C::THREADS);
-  cfg.dynamicSmemBytes = C::SMEM_BYTES;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[1];
-  cfg.attrs = attr;
-  cfg.numAttrs = 0;
-  if (gemm_pdl_enabled()) {
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.numAttrs = 1;
-  }
-  cudaError_t e = cudaLaunchKernelEx(&cfg, kern, ta4, tb4, ta8, tb8, args);
-  if (e != cudaSuccess) return fail(ATOM_E_CUDA, "gemm_i4 (wide) launch: %s", cudaGetErrorString(e));
-  return ATOM_OK;
+  const dim3 grid((unsigned)((op.N + C::BN - 1) / C::BN), (unsigned)((op.M + C::BM - 1) / C::BM), 1);
+  return launch("gemm_i4 (tall)", kern, grid, dim3(C::THREADS), C::SMEM_BYTES, stream, 0, gemm_pdl_enabled(), tp4, tq4, tp8, tq8, args);
 }
 
 template <bool kO4, bool kPush = false>
@@ -396,22 +325,15 @@ int gemm_dispatch(const GemmOperands& op, const atom::GemmArgs& args, uint32_t f
   // (65..128 tokens are two 64-token tiles per channel tile: only while those CTAs still fit one wave of 148 SMs)
   const bool skinny = (flags & ATOM_GEMM_FORCE_SKINNY) ||
                       (!(flags & ATOM_GEMM_FORCE_TALL) && (op.M <= 64 || (op.M <= 128 && (op.N + 127) / 128 * 2 <= 148)));
-  // <swap, BN, groups per pipeline stage, packed stages, K split, o4, converter warps, epilogue warpgroups>
-  if (!skinny) {
-    if (flags & ATOM_GEMM_LEGACY_TALL) return launch_gemm<false, 128, 2, 2, 1, kO4, 4, 2>(op, args, stream);
-    // 128 x 128 tiles by default.  The 128 x 256 kernel (token operand in tensor memory) halves the token-side conversion
-    // per MMA but measured slower at every size (4096^3: 704 vs 783-829 TOP/s, its 128-accumulator epilogue spills), so it
-    // only runs on request.
-    return (flags & ATOM_GEMM_FORCE_WIDE) ? launch_wide<kO4>(op, args, stream) : launch_tall<kO4>(op, args, stream);
-  }
-  // 33..64 tokens: the round-1 configuration (one CTA per SM, 8 converter warps) still measures faster than the new
-  // kernel's BN=64 instance (4096^2: 13.0-13.3 vs 15.0 us), which then only runs on request and under the fused epilogues
-  if (op.M <= 64 && !(flags & ATOM_GEMM_LEGACY_SKINNY) && (op.M <= 32 || (flags & ATOM_GEMM_FORCE_SKINNY))) {
+  if (!skinny) return launch_tall<kO4>(op, args, stream);
+  // up to 32 tokens, or on request up to 64: the decode kernel
+  if (op.M <= 32 || (op.M <= 64 && (flags & ATOM_GEMM_FORCE_SKINNY))) {
     if constexpr (!kO4) { if (args.ar.bufs != nullptr) return skinny_dispatch<false, true>(op, args, flags, stream); }
     return skinny_dispatch<kO4>(op, args, flags, stream);
   }
-  // decode shapes: weights on the MMA-M axis; K split 4-way over a cluster when one wave of CTAs would not
-  // cover the machine (the kernel is HBM-bound on the weights: more CTAs = more bytes in flight)
+  // from 33 tokens on: the weight-stationary kernel (one CTA per SM, 8 converter warps, 64-token tiles) still measures
+  // faster than the decode kernel's BN=64 instance (4096^2: 13.0-13.3 vs 15.0 us).  K split 4-way over a cluster when one
+  // wave of CTAs would not cover the machine (the kernel is HBM-bound on the weights: more CTAs = more bytes in flight)
   const int64_t ch_tiles = (op.N + 127) / 128;
   const int groups = args.G + 1;
   // K split over a cluster (1, 2 or 4 ranks): as many CTAs as it takes to give every SM about one, no more -- each extra
@@ -420,24 +342,25 @@ int gemm_dispatch(const GemmOperands& op, const atom::GemmArgs& args, uint32_t f
   int ksplit = 1;
   // o4 quantises from the FP32 sums: a K split would reorder them and move INT4 codes by one, so the KV projections
   // never split (bit-identical codes to the reference kernel on every path)
-  if (!kO4 && !(flags & ATOM_GEMM_NO_SPLITK) && groups >= 8) {
-    if (flags & ATOM_GEMM_SPLITK2) ksplit = 2;
-    else if (flags & ATOM_GEMM_SPLITK4) ksplit = 4;
-    else ksplit = tiles * 4 <= 148 ? 4 : (tiles * 2 <= 148 ? 2 : 1);   // the largest split that still fits one wave of 148 SMs
+  if constexpr (!kO4) {
+    if (!(flags & ATOM_GEMM_NO_SPLITK) && groups >= 8) {
+      if (flags & ATOM_GEMM_SPLITK2) ksplit = 2;
+      else if (flags & ATOM_GEMM_SPLITK4) ksplit = 4;
+      else ksplit = tiles * 4 <= 148 ? 4 : (tiles * 2 <= 148 ? 2 : 1);   // the largest split that still fits one wave of 148 SMs
+    }
+    // <groups per pipeline stage, packed stages, K split, o4>
+    if (ksplit == 4) return launch_gemm<1, 4, 4, false>(op, args, stream);
+    if (ksplit == 2) return launch_gemm<2, 2, 2, false>(op, args, stream);
   }
-#define ATOM_SKINNY(BN, GS4, GS2, GS1, KP4, KP2, KP1, EW)                                                      \
-  return ksplit == 4   ? launch_gemm<true, BN, GS4, KP4, 4, kO4, 8, EW>(op, args, stream)                      \
-         : ksplit == 2 ? launch_gemm<true, BN, GS2, KP2, 2, kO4, 8, EW>(op, args, stream)                      \
-                       : launch_gemm<true, BN, GS1, KP1, 1, kO4, 8, EW>(op, args, stream)
-  if (op.M <= 16) { ATOM_SKINNY(16, 2, 2, 2, 4, 4, 4, 1); }
-  if (op.M <= 32) { ATOM_SKINNY(32, 2, 2, 2, 4, 4, 4, 1); }
-  ATOM_SKINNY(64, 1, 2, 2, 4, 2, 3, 2);
-#undef ATOM_SKINNY
+  return launch_gemm<2, 3, 1, kO4>(op, args, stream);
 }
 
 int gemm_common(const void* a, const void* b, const void* a_scale, const void* b_scale, const void* a_keeper,
                 const void* b_keeper, const void* a_keeper_scale, const void* b_keeper_scale, void* d, void* d_scale,
                 int64_t M, int64_t N, int64_t K, uint32_t flags, void* stream, bool o4, const atom::ArArgs* ar = nullptr) {
+  constexpr uint32_t known = ATOM_GEMM_NO_SPLITK | ATOM_GEMM_FORCE_TALL | ATOM_GEMM_FORCE_SKINNY | ATOM_GEMM_SPLITK2 |
+                             ATOM_GEMM_SPLITK4 | ATOM_GEMM_SPLITK8;
+  ATOM_REQUIRE((flags & ~known) == 0, "gemm_i4: unknown flags 0x%x (known: 0x%x)", flags & ~known, known);
   ATOM_REQUIRE(a && b && a_scale && b_scale && a_keeper && b_keeper && a_keeper_scale && b_keeper_scale && (d || ar),
                "gemm_i4: null pointer argument");
   ATOM_REQUIRE(M > 0 && N > 0, "gemm_i4: M=%lld N=%lld must be positive", (long long)M, (long long)N);
@@ -451,7 +374,7 @@ int gemm_common(const void* a, const void* b, const void* a_scale, const void* b
     ATOM_REQUIRE(ar->bufs && ar->state && ar->world >= 1 && ar->world <= 32 && ar->rank >= 0 && ar->rank < ar->world && ar->slot % 8 == 0 &&
                  M * N <= ar->slot, "gemm_i4_o16_push: rank=%d world=%d, M x N = %lld must fit a slot of %lld elements", ar->rank, ar->world,
                  (long long)(M * N), (long long)ar->slot);
-    flags = (flags | ATOM_GEMM_FORCE_SKINNY) & ~(ATOM_GEMM_FORCE_TALL | ATOM_GEMM_LEGACY_SKINNY);
+    flags = (flags | ATOM_GEMM_FORCE_SKINNY) & ~ATOM_GEMM_FORCE_TALL;
   }
   ATOM_REQUIRE(aligned16(b_scale) && aligned16(b_keeper_scale), "gemm_i4: weight scale pointers must be 16-byte aligned");
   ATOM_REQUIRE((reinterpret_cast<uintptr_t>(a_scale) & 3) == 0 && (reinterpret_cast<uintptr_t>(a_keeper_scale) & 3) == 0,
@@ -479,7 +402,7 @@ int quant_check(const char* what, int seq_len, int hidden, const void* o8, const
 
 extern "C" {
 
-int atom_version(void) { return 100; }
+int atom_version(void) { return 101; }
 const char* atom_last_error(void) { return g_err.c_str(); }
 int atom_scale_index(int row) { return atom::scale_index(row); }
 int atom_scale_size(int rows) { return atom::scale_size(rows); }

@@ -20,9 +20,11 @@
 // every commit therefore covers GS groups; one commit per stage serves both the epilogue ("accumulators ready") and
 // the converter ("operand slot free").
 //
-// kSwap=false ("tall"):   MMA-M = 128 tokens (A), MMA-N = BN output channels (B).
-// kSwap=true  ("skinny"): MMA-M = 128 output channels (B), MMA-N = BN tokens (A) -- decode shapes;
-//       optionally split along K over a thread-block cluster, partial sums pushed into the leader through DSMEM.
+// Weight-stationary: MMA-M = 128 output channels (B), MMA-N = BN = 64 tokens (A), 8 converter warps, 2 epilogue
+// warpgroups.  gemm_dispatch runs it for 33-128 tokens; optionally split along K over a thread-block cluster, partial
+// sums pushed into the leader through DSMEM.
+//
+// GemmArgs, expand_chunk, convert_tile, the scale layout and trace_stamp are shared with the decode and 128x128 kernels.
 #pragma once
 #include "ptx_sm100.cuh"
 
@@ -72,17 +74,18 @@ __device__ __forceinline__ float silu_ref(float x) { return x / (1.0f + expf(-x)
 __host__ __device__ __forceinline__ int scale_index(int row) { return (row / 16) * 64 + (row % 8) * 8 + ((row / 8) % 2); }
 __host__ __device__ __forceinline__ int scale_size(int m) { return m / 16 * 64 + 64 - (1 - (m % 16) / 8) * (8 - (m % 8)) * 8; }
 
-template <bool kSwap, int BN, int GS, int kPack, int kSplit, bool kO4, int kConvWarps, int kEpiWgs>
+template <int GS, int kPack, int kSplit, bool kO4>
 struct GemmCfg {
-  static constexpr int BM = 128;                                  // MMA M (TMEM lanes)
+  static constexpr int BM = 128;                                  // MMA M (TMEM lanes) = output channels per tile
+  static constexpr int BN = 64;                                   // MMA N = tokens per tile
   static constexpr int RING = 2;                                  // operand-slot / accumulator stages
   static constexpr int TMEM_COLS_RAW = RING * GS * BN;
   static constexpr int TMEM_COLS = TMEM_COLS_RAW <= 32 ? 32 : (TMEM_COLS_RAW <= 64 ? 64 : (TMEM_COLS_RAW <= 128 ? 128 : (TMEM_COLS_RAW <= 256 ? 256 : 512)));
   static constexpr int SCALE_STAGES = 4;                          // scale ring depth, in stages
   static constexpr int SCALE_GROUP_BYTES = 512;                   // 256 B MMA-M side + 256 B MMA-N side, raw copies
-  static constexpr int EPI_WGS = kEpiWgs;                         // epilogue warpgroups (each owns BN/EPI_WGS columns)
+  static constexpr int EPI_WGS = 2;                               // epilogue warpgroups (each owns BN/EPI_WGS columns)
   static constexpr int CPT = BN / EPI_WGS;                        // accumulator columns per epilogue thread
-  static constexpr int CONV_WARPS = kConvWarps;
+  static constexpr int CONV_WARPS = 8;
   static constexpr int CONV_THREADS = CONV_WARPS * 32;
   static constexpr int THREADS = 256 + 128 * EPI_WGS + (CONV_WARPS - 4) * 32;   // extra converters sit after the epilogue
   static constexpr int PACK_P = BM * 64, PACK_Q = BN * 64;        // bytes per packed group
@@ -98,10 +101,7 @@ struct GemmCfg {
   static constexpr int NUM_BARS = 2 * kPack + 3 * RING + 2 * SCALE_STAGES;
   static constexpr int OFF_TMEM_PTR = OFF_BAR + NUM_BARS * 8;
   static constexpr int SMEM_BYTES = OFF_TMEM_PTR + 16 + 1024;     // + slack for the 1024-B alignment fix-up
-  static_assert(!kO4 || (BN == 128 || kSwap), "o4 (tall) quantises one 128-column head per CTA");
   static_assert(SMEM_BYTES <= 227 * 1024, "shared memory budget");
-  static_assert(BN <= 128, "scale slot holds 128 channel scales");
-  static_assert(CPT % 16 == 0 && CPT >= 16, "epilogue column slices are multiples of 16");
   static_assert(TMEM_COLS_RAW <= 512, "TMEM has 512 columns");
 };
 
@@ -141,14 +141,15 @@ __device__ __forceinline__ void convert_tile(const uint8_t* __restrict__ packed,
   }
 }
 
-template <bool kSwap, int BN, int GS, int kPack, int kSplit, bool kO4, int kConvWarps, int kEpiWgs>
-__global__ void __launch_bounds__(GemmCfg<kSwap, BN, GS, kPack, kSplit, kO4, kConvWarps, kEpiWgs>::THREADS, 1)
-gemm_i4_kernel(const __grid_constant__ CUtensorMap tm_p4,   // packed INT4, MMA-M operand  (box 64 B x 128 rows)
-               const __grid_constant__ CUtensorMap tm_q4,   // packed INT4, MMA-N operand  (box 64 B x BN rows)
-               const __grid_constant__ CUtensorMap tm_p8,   // INT8 keeper, MMA-M operand  (box 128 B x 128 rows, SW128)
-               const __grid_constant__ CUtensorMap tm_q8,   // INT8 keeper, MMA-N operand  (box 128 B x BN rows, SW128)
+template <int GS, int kPack, int kSplit, bool kO4>
+__global__ void __launch_bounds__(GemmCfg<GS, kPack, kSplit, kO4>::THREADS, 1)
+gemm_i4_kernel(const __grid_constant__ CUtensorMap tm_p4,   // packed INT4 weights      (box 64 B x 128 rows)
+               const __grid_constant__ CUtensorMap tm_q4,   // packed INT4 tokens       (box 64 B x BN rows)
+               const __grid_constant__ CUtensorMap tm_p8,   // INT8 keeper, weights     (box 128 B x 128 rows, SW128)
+               const __grid_constant__ CUtensorMap tm_q8,   // INT8 keeper, tokens      (box 128 B x BN rows, SW128)
                const GemmArgs args) {
-  using C = GemmCfg<kSwap, BN, GS, kPack, kSplit, kO4, kConvWarps, kEpiWgs>;
+  using C = GemmCfg<GS, kPack, kSplit, kO4>;
+  constexpr int BN = C::BN;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   // 1024-B alignment (SWIZZLE_128B atoms) by offsetting the shared array, NOT by integer-casting the pointer:
   // an integer round trip makes the compiler fall back to generic LD/ST for every smem access.
@@ -167,9 +168,9 @@ gemm_i4_kernel(const __grid_constant__ CUtensorMap tm_p4,   // packed INT4, MMA-
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   // blockIdx.x = output-channel tile: CTAs launched together share the token tile (L2) and stream disjoint weights
   const int tile_ch = blockIdx.x, tile_tok = blockIdx.y;
-  const int p0 = (kSwap ? tile_ch : tile_tok) * C::BM;   // first row of the MMA-M operand
-  const int q0 = (kSwap ? tile_tok : tile_ch) * BN;      // first row of the MMA-N operand
-  const int m0 = kSwap ? q0 : p0, n0 = kSwap ? p0 : q0;  // token / channel origin of the tile
+  const int p0 = tile_ch * C::BM;                        // first row of the MMA-M operand (weights)
+  const int q0 = tile_tok * BN;                          // first row of the MMA-N operand (tokens)
+  const int m0 = q0, n0 = p0;                            // token / channel origin of the tile
 
   // K split over the cluster: groups [g_begin, g_end) of the G+1 groups (index G = INT8 keeper)
   const int total_groups = args.G + 1;
@@ -198,7 +199,7 @@ gemm_i4_kernel(const __grid_constant__ CUtensorMap tm_p4,   // packed INT4, MMA-
   auto issue_stage = [&](int s, int ps, int part = 0) {
     const int n4 = stage_int4(s);
     if (part != 2) mbar_arrive_expect_tx(&pack_full[ps], n4 * (C::PACK_P + C::PACK_Q));
-    const bool do_p = part == 0 || (part == 1) == kSwap, do_q = part == 0 || (part == 1) != kSwap;   // kSwap: P = weights
+    const bool do_p = part != 2, do_q = part != 1;      // P = weights, Q = activations
     for (int j = 0; j < n4; ++j) {
       const int g = g_begin + s * GS + j;
       if (do_p) tma_load_2d(smem + C::OFF_PACK_P + (ps * GS + j) * C::PACK_P, &tm_p4, &pack_full[ps], g * 64, p0);
@@ -274,9 +275,8 @@ gemm_i4_kernel(const __grid_constant__ CUtensorMap tm_p4,   // packed INT4, MMA-
     // ============================================================ scale loader: cp.async straight into the scale ring,
     // completion counted on scale_full by the copy engine -- no thread ever waits on a scale's DRAM latency.
     // Group slot layout (raw copies of the reference layouts):
-    //   [0,256)   MMA-M side: tall  -> 64 (lower,upper) half2 words of the A-scale rows   (word = (r/16)*8 + r%8)
-    //                          skinny-> 128 B-scale halves of the channel tile (thread n reads the pair word n/2)
-    //   [256,512) MMA-N side: tall  -> BN B-scale halves;  skinny -> BN/16*8 (lower,upper) words of the token rows
+    //   [0,256)   MMA-M side: 128 B-scale halves of the channel tile (thread n reads the pair word n/2)
+    //   [256,512) MMA-N side: BN/16*8 (lower,upper) A-scale words of the token rows
     if (args.pdl) griddep_wait();           // the activation scales are the preceding kernel's output
     for (int s = 0; s < nstages; ++s) {
       const int ss = s % C::SCALE_STAGES;
@@ -288,9 +288,9 @@ gemm_i4_kernel(const __grid_constant__ CUtensorMap tm_p4,   // packed INT4, MMA-
         const __half* as_row = keeper ? args.a_keeper_scale : args.a_scale + (size_t)g * args.lda_scale;
         const __half* bs_row = keeper ? args.b_keeper_scale : args.b_scale + (size_t)g * args.N;
         uint8_t* slot_p = smem + C::OFF_SM + (ss * GS + j) * C::SCALE_GROUP_BYTES;
-        constexpr int TOK = kSwap ? BN : C::BM, CHN = kSwap ? C::BM : BN;
-        uint8_t* tok_dst = slot_p + (kSwap ? 256 : 0);
-        uint8_t* chn_dst = slot_p + (kSwap ? 0 : 256);
+        constexpr int TOK = BN, CHN = C::BM;
+        uint8_t* tok_dst = slot_p + 256;
+        uint8_t* chn_dst = slot_p;
 #pragma unroll
         for (int w = lane; w < TOK / 2; w += 32) {              // A-scale words: rows (16 blk + i, 16 blk + i + 8)
           const int blk = w >> 3, i = w & 7;
@@ -347,8 +347,6 @@ gemm_i4_kernel(const __grid_constant__ CUtensorMap tm_p4,   // packed INT4, MMA-
     float acc[C::CPT];
 #pragma unroll
     for (int i = 0; i < C::CPT; ++i) acc[i] = 0.f;
-    const bool upper = kSwap ? false : (((m0 + row) & 15) >= 8);
-    const uint32_t pair_sel = upper ? 0x7632u : 0x5410u;   // one PRMT picks the odd (upper rows) or even channel of two pairs
 
     for (int s = 0; s < nstages; ++s) {
       const int es = s % C::RING, ss = s % C::SCALE_STAGES;
@@ -360,19 +358,9 @@ gemm_i4_kernel(const __grid_constant__ CUtensorMap tm_p4,   // packed INT4, MMA-
       for (int j = 0; j < ng; ++j) {
         const bool keeper = (g_begin + s * GS + j == args.G);
         const uint8_t* slot_p = smem + C::OFF_SM + (ss * GS + j) * C::SCALE_GROUP_BYTES;
-        __half2 sm2;
-        const __half* sn;      // tall: B-scale halves of this thread's columns
-        const __half2* snw;    // skinny: (lower, upper) A-scale words of this thread's token columns
-        if constexpr (!kSwap) {
-          const __half2 pw = reinterpret_cast<const __half2*>(slot_p)[(row >> 4) * 8 + (row & 7)];
-          sm2 = __half2half2(upper ? __high2half(pw) : __low2half(pw));
-          sn = reinterpret_cast<const __half*>(slot_p + 256) + colbase;
-          snw = nullptr;
-        } else {
-          sm2 = reinterpret_cast<const __half2*>(slot_p)[row >> 1];     // {sB[n&~1], sB[n|1]}
-          sn = nullptr;
-          snw = reinterpret_cast<const __half2*>(slot_p + 256) + (colbase >> 4) * 8;
-        }
+        const __half2 sm2 = reinterpret_cast<const __half2*>(slot_p)[row >> 1];     // {sB[n&~1], sB[n|1]}
+        // (lower, upper) A-scale words of this thread's token columns
+        const __half2* snw = reinterpret_cast<const __half2*>(slot_p + 256) + (colbase >> 4) * 8;
         const uint32_t taddr = tmem_base + ((uint32_t)(wq * 32) << 16) + (uint32_t)((es * GS + j) * BN + colbase);
         constexpr int CH = (C::CPT >= 32) ? 32 : 16;
 #pragma unroll
@@ -390,32 +378,16 @@ gemm_i4_kernel(const __grid_constant__ CUtensorMap tm_p4,   // packed INT4, MMA-
 #pragma unroll
             for (int i = 0; i < CH; ++i) r[i] = (uint32_t)((int32_t)r[i] << 8);
           }
-          if constexpr (!kSwap) {
-            // thread = token row; columns = channels.  rs is shared by the column pair (2p, 2p+1).
+          // thread = channel row (sm2 = {sB[n&~1], sB[n|1]}); columns = tokens, 16-aligned tile origin:
+          // token i with i%16<8 pairs with sm2.x, i%16>=8 with sm2.y
 #pragma unroll
-            for (int p = 0; p < CH / 2; p += 2) {
-              const __half2 n01 = *reinterpret_cast<const __half2*>(sn + c0 + 2 * p);
-              const __half2 n23 = *reinterpret_cast<const __half2*>(sn + c0 + 2 * p + 2);
-              const uint32_t selw = __byte_perm(*reinterpret_cast<const uint32_t*>(&n01), *reinterpret_cast<const uint32_t*>(&n23), pair_sel);
-              const __half2 sel = *reinterpret_cast<const __half2*>(&selw);   // {sB[pair p], sB[pair p+1]} for this row's half
-              const float2 rs = __half22float2(__hmul2(sm2, sel));
-              acc[c0 + 2 * p + 0] = fmaf((float)(int32_t)r[2 * p + 0], rs.x, acc[c0 + 2 * p + 0]);
-              acc[c0 + 2 * p + 1] = fmaf((float)(int32_t)r[2 * p + 1], rs.x, acc[c0 + 2 * p + 1]);
-              acc[c0 + 2 * p + 2] = fmaf((float)(int32_t)r[2 * p + 2], rs.y, acc[c0 + 2 * p + 2]);
-              acc[c0 + 2 * p + 3] = fmaf((float)(int32_t)r[2 * p + 3], rs.y, acc[c0 + 2 * p + 3]);
-            }
-          } else {
-            // thread = channel row (sm2 = {sB[n&~1], sB[n|1]}); columns = tokens, 16-aligned tile origin:
-            // token i with i%16<8 pairs with sm2.x, i%16>=8 with sm2.y
+          for (int q = 0; q < CH; q += 16) {
 #pragma unroll
-            for (int q = 0; q < CH; q += 16) {
-#pragma unroll
-              for (int i = 0; i < 8; ++i) {
-                const __half2 a2 = snw[((c0 + q) >> 4) * 8 + i];      // (sA[token q+i], sA[token q+i+8])
-                const float2 rs = __half22float2(__hmul2(a2, sm2));
-                acc[c0 + q + i] = fmaf((float)(int32_t)r[q + i], rs.x, acc[c0 + q + i]);
-                acc[c0 + q + i + 8] = fmaf((float)(int32_t)r[q + i + 8], rs.y, acc[c0 + q + i + 8]);
-              }
+            for (int i = 0; i < 8; ++i) {
+              const __half2 a2 = snw[((c0 + q) >> 4) * 8 + i];      // (sA[token q+i], sA[token q+i+8])
+              const float2 rs = __half22float2(__hmul2(a2, sm2));
+              acc[c0 + q + i] = fmaf((float)(int32_t)r[q + i], rs.x, acc[c0 + q + i]);
+              acc[c0 + q + i + 8] = fmaf((float)(int32_t)r[q + i + 8], rs.y, acc[c0 + q + i + 8]);
             }
           }
         }
@@ -451,100 +423,45 @@ gemm_i4_kernel(const __grid_constant__ CUtensorMap tm_p4,   // packed INT4, MMA-
     if (kSplit == 1 || krank == 0) {
       constexpr float kInv = 1.0f / 256.0f;   // exact: removes the 16*16 operand factor
       if constexpr (!kO4) {
-        if constexpr (!kSwap) {
-          const int m = m0 + row;
-          if (m < args.M) {
-            __half* drow = args.d + (size_t)m * args.N + n0 + colbase;
+        const int n = n0 + row;
+        if (n < args.N) {
 #pragma unroll
-            for (int i = 0; i < C::CPT; i += 8) {
-              if (n0 + colbase + i < args.N) {   // N is a multiple of 8 (16-B rows)
-                uint4 v;
-                __half2 h0 = __floats2half2_rn(acc[i + 0] * kInv, acc[i + 1] * kInv);
-                __half2 h1 = __floats2half2_rn(acc[i + 2] * kInv, acc[i + 3] * kInv);
-                __half2 h2 = __floats2half2_rn(acc[i + 4] * kInv, acc[i + 5] * kInv);
-                __half2 h3 = __floats2half2_rn(acc[i + 6] * kInv, acc[i + 7] * kInv);
-                v.x = *reinterpret_cast<uint32_t*>(&h0); v.y = *reinterpret_cast<uint32_t*>(&h1);
-                v.z = *reinterpret_cast<uint32_t*>(&h2); v.w = *reinterpret_cast<uint32_t*>(&h3);
-                *reinterpret_cast<uint4*>(drow + i) = v;
-              }
-            }
-          }
-        } else {
-          const int n = n0 + row;
-          if (n < args.N) {
-#pragma unroll
-            for (int i = 0; i < C::CPT; ++i) {
-              const int m = m0 + colbase + i;
-              if (m < args.M) args.d[(size_t)m * args.N + n] = __float2half_rn(acc[i] * kInv);   // warp writes 64 B runs
-            }
+          for (int i = 0; i < C::CPT; ++i) {
+            const int m = m0 + colbase + i;
+            if (m < args.M) args.d[(size_t)m * args.N + n] = __float2half_rn(acc[i] * kInv);   // warp writes 64 B runs
           }
         }
       } else {
         // o4 epilogue (DenseLayerGEMM_i4_o4.cu:705-787): per (token, 128-channel head) asymmetric INT4 with the
-        // reference's |v| min/max.  tall: two epilogue WGs hold 64 columns each of the same row.
+        // reference's |v| min/max.  Thread = channel; reduce |v| min/max over the 128 channels of the head for every
+        // token column.
         float* xch = reinterpret_cast<float*>(smem + C::OFF_PACK_P);   // packed ring is idle by now
-        if constexpr (!kSwap) {
-          float mx = -INFINITY, mn = INFINITY;
+        float* xmx = xch;                 // [4 warps][BN]
+        float* xmn = xch + 4 * BN;
+        const int ewarp = warp - 8;       // each of the 2 WGs owns CPT token columns
 #pragma unroll
-          for (int i = 0; i < C::CPT; ++i) { acc[i] *= kInv; const float a = fabsf(acc[i]); mx = fmaxf(mx, a); mn = fminf(mn, a); }
-          const int part = (warp - 8) >> 2;          // which column slice of the 128-channel head this warpgroup holds
-          xch[(part * 2 + 0) * C::BM + row] = mx;
-          xch[(part * 2 + 1) * C::BM + row] = mn;
-          asm volatile("bar.sync 1, %0;" ::"n"(128 * C::EPI_WGS) : "memory");
+        for (int i = 0; i < C::CPT; ++i) {
+          acc[i] *= kInv;
+          // |v| >= 0: IEEE bit patterns order like unsigned integers, so one REDUX each replaces 5 shuffle rounds
+          uint32_t ua = __float_as_uint(fabsf(acc[i])), umx = ua, umn = ua;
+          if (n0 + row >= args.N) { umx = 0u; umn = 0x7f800000u; }
+          umx = __reduce_max_sync(0xffffffffu, umx);
+          umn = __reduce_min_sync(0xffffffffu, umn);
+          if (lane == 0) { xmx[(ewarp & 3) * BN + colbase + i] = __uint_as_float(umx); xmn[(ewarp & 3) * BN + colbase + i] = __uint_as_float(umn); }
+        }
+        asm volatile("bar.sync 1, %0;" ::"n"(128 * C::EPI_WGS) : "memory");
+        const int n = n0 + row;
 #pragma unroll
-          for (int o = 0; o < C::EPI_WGS; ++o) {
-            mx = fmaxf(mx, xch[(o * 2 + 0) * C::BM + row]);
-            mn = fminf(mn, xch[(o * 2 + 1) * C::BM + row]);
-          }
+        for (int i = 0; i < C::CPT; ++i) {
+          const int c = colbase + i, m = m0 + c;
+          const float mx = fmaxf(fmaxf(xmx[c], xmx[BN + c]), fmaxf(xmx[2 * BN + c], xmx[3 * BN + c]));
+          const float mn = fminf(fminf(xmn[c], xmn[BN + c]), fminf(xmn[2 * BN + c], xmn[3 * BN + c]));
           const float scale = (mx - mn) / 15.f, zero = -mn, r_scale = 1.f / scale;
-          const int m = m0 + row;
-          if (m < args.M) {
-            if (part == 0) args.d_scale[(size_t)m * (args.N / 128) + tile_ch] = __floats2half2_rn(scale, zero);
-            uint32_t pk[C::CPT / 8];
-#pragma unroll
-            for (int i = 0; i < C::CPT; i += 8) {
-              uint32_t w = 0;
-#pragma unroll
-              for (int e = 0; e < 8; ++e) w |= ((uint32_t)((int)roundf((acc[i + e] + zero) * r_scale) & 0xF)) << (4 * e);
-              pk[i / 8] = w;
-            }
-            uint4* dst = reinterpret_cast<uint4*>(args.d4 + (size_t)m * (args.N / 2) + (n0 + colbase) / 2);
-            if constexpr (C::CPT >= 32) {
-#pragma unroll
-              for (int i = 0; i < C::CPT / 32; ++i) dst[i] = make_uint4(pk[4 * i], pk[4 * i + 1], pk[4 * i + 2], pk[4 * i + 3]);
-            } else {
-              *reinterpret_cast<uint2*>(dst) = make_uint2(pk[0], pk[1]);
-            }
-          }
-        } else {
-          // skinny: thread = channel; reduce |v| min/max over the 128 channels of the head for every token column
-          float* xmx = xch;                 // [4 warps][BN]
-          float* xmn = xch + 4 * BN;
-          const int ewarp = warp - 8;       // EPI_WGS == 1 or 2; with 2 WGs each owns CPT token columns
-#pragma unroll
-          for (int i = 0; i < C::CPT; ++i) {
-            acc[i] *= kInv;
-            // |v| >= 0: IEEE bit patterns order like unsigned integers, so one REDUX each replaces 5 shuffle rounds
-            uint32_t ua = __float_as_uint(fabsf(acc[i])), umx = ua, umn = ua;
-            if (n0 + row >= args.N) { umx = 0u; umn = 0x7f800000u; }
-            umx = __reduce_max_sync(0xffffffffu, umx);
-            umn = __reduce_min_sync(0xffffffffu, umn);
-            if (lane == 0) { xmx[(ewarp & 3) * BN + colbase + i] = __uint_as_float(umx); xmn[(ewarp & 3) * BN + colbase + i] = __uint_as_float(umn); }
-          }
-          asm volatile("bar.sync 1, %0;" ::"n"(128 * C::EPI_WGS) : "memory");
-          const int n = n0 + row;
-#pragma unroll
-          for (int i = 0; i < C::CPT; ++i) {
-            const int c = colbase + i, m = m0 + c;
-            const float mx = fmaxf(fmaxf(xmx[c], xmx[BN + c]), fmaxf(xmx[2 * BN + c], xmx[3 * BN + c]));
-            const float mn = fminf(fminf(xmn[c], xmn[BN + c]), fminf(xmn[2 * BN + c], xmn[3 * BN + c]));
-            const float scale = (mx - mn) / 15.f, zero = -mn, r_scale = 1.f / scale;
-            int q = (int)roundf((acc[i] + zero) * r_scale) & 0xF;
-            const int qn = __shfl_down_sync(0xffffffffu, q, 1);     // channel n+1 lives in the next lane
-            if (m < args.M && n < args.N) {
-              if ((lane & 1) == 0) args.d4[(size_t)m * (args.N / 2) + n / 2] = (uint8_t)(q | (qn << 4));
-              if (row == 0) args.d_scale[(size_t)m * (args.N / 128) + tile_ch] = __floats2half2_rn(scale, zero);
-            }
+          int q = (int)roundf((acc[i] + zero) * r_scale) & 0xF;
+          const int qn = __shfl_down_sync(0xffffffffu, q, 1);     // channel n+1 lives in the next lane
+          if (m < args.M && n < args.N) {
+            if ((lane & 1) == 0) args.d4[(size_t)m * (args.N / 2) + n / 2] = (uint8_t)(q | (qn << 4));
+            if (row == 0) args.d_scale[(size_t)m * (args.N / 128) + tile_ch] = __floats2half2_rn(scale, zero);
           }
         }
       }

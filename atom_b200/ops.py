@@ -17,9 +17,6 @@ __all__ = [
 
 GEMM_AUTO, GEMM_NO_SPLITK, GEMM_FORCE_TALL, GEMM_FORCE_SKINNY = 0, 1, 2, 4
 GEMM_SPLITK2, GEMM_SPLITK4 = 16, 32
-GEMM_FORCE_WIDE, GEMM_NO_WIDE = 512, 1024   # prefill shapes: 128 x 256 tiles with the token operand in tensor memory / never
-GEMM_LEGACY_TALL = 256    # prefill shapes: the round-1 kernel, kept for A/B timing
-GEMM_LEGACY_SKINNY = 128  # decode shapes: the round-1 kernel, kept for A/B timing
 
 
 def _stream(t):

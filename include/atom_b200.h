@@ -43,10 +43,7 @@ extern "C" {
 #define ATOM_GEMM_SPLITK2 16u     /* decode shapes: force a 2-way K split (default: chosen from the tile count) */
 #define ATOM_GEMM_SPLITK4 32u     /* decode shapes: force a 4-way K split */
 #define ATOM_GEMM_SPLITK8 64u     /* decode shapes, M <= 32: force an 8-way K split (cluster of 8) */
-#define ATOM_GEMM_FORCE_WIDE 512u    /* prefill shapes: 128 x 256 tiles, token operand in tensor memory (opt-in: measured slower than 128 x 128) */
-#define ATOM_GEMM_NO_WIDE 1024u      /* prefill shapes: always 128 x 128 tiles (the default; kept for callers that pass it) */
-#define ATOM_GEMM_LEGACY_TALL 256u   /* prefill shapes: the round-1 kernel (I2F + FFMA epilogue), kept for A/B timing */
-#define ATOM_GEMM_LEGACY_SKINNY 128u /* decode shapes: the round-1 kernel (weights expanded into shared memory), kept for A/B timing */
+/* atom_gemm_i4_o16, atom_gemm_i4_o16_push and atom_gemm_i4_o4 reject any other bit with ATOM_E_INVALID */
 
 ATOM_API int atom_version(void);
 ATOM_API const char* atom_last_error(void);

@@ -111,10 +111,9 @@ GEMM_CASES = [
     (64, 384, 4096, 5, True), (16, 4096, 4096, 1, True),
     (16, 4096, 4096, 0, False), (32, 1024, 4096, 0, False), (48, 512, 11008, 0, False), (5, 128, 2048, 0, False),
     (130, 2752, 1024, 0, True), (100, 256, 2048, 0, False), (128, 512, 512, 1, True), (65, 1024, 4096, 1, True),
-    # 512 = 128 x 256 tiles with the token operand in tensor memory (the default once such tiles fill the GPU): N % 256 != 0
-    # (one-half last tile, partially filled second half), M tails, long K
-    (300, 256, 4096, 512, True), (129, 384, 1024, 512, True), (130, 2752, 1024, 512, True), (7, 512, 384, 512, True),
-    (1000, 1024, 2048, 1024, True),
+    # the 128 x 128 prefill kernel, by default (M > 128) or forced: N % 256 != 0, M tails, long K
+    (300, 256, 4096, 0, True), (129, 384, 1024, 0, True), (130, 2752, 1024, 2, True), (7, 512, 384, 2, True),
+    (1000, 1024, 2048, 0, True),
 ]
 
 
@@ -135,7 +134,7 @@ def test_gemm_o16(m, n, k, flags, exact):
 
 
 @pytest.mark.parametrize("m,n,k,flags", [(16, 256, 512, 2), (130, 384, 1024, 2), (16, 256, 512, 5), (7, 128, 1024, 5),
-                                         (48, 4096, 4096, 1), (16, 4096, 4096, 1), (130, 384, 1024, 512), (300, 512, 2048, 512)])
+                                         (48, 4096, 4096, 1), (16, 4096, 4096, 1), (130, 384, 1024, 0), (300, 512, 2048, 0)])
 def test_gemm_o4(m, n, k, flags):
     from atom_b200 import ops
     t = O.make_gemm_inputs(m, n, k, seed=m + n + k)

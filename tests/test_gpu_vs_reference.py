@@ -30,9 +30,7 @@ GEMM_O16_CASES = [(16, 4096, 4096, 1), (7, 4096, 4096, 1), (128, 4096, 4096, 1),
                   (32, 5120, 5120, 1), (32, 13824, 5120, 1), (32, 5120, 13824, 1), (32, 1024, 8192, 1),
                   (32, 8192, 2816, 1), (32, 8192, 2688, 1), (64, 8192, 1024, 1),
                   # prefill: the 7B MLP up-projection and config #3's 16 x 2048 tokens
-                  (4096, 11008, 4096, 0), (32768, 4096, 4096, 0),
-                  # the same prefill shapes forced through each of the two prefill kernels
-                  (4096, 4096, 4096, 512), (4096, 4096, 4096, 1024), (1000, 11008, 4096, 512)]
+                  (4096, 11008, 4096, 0), (32768, 4096, 4096, 0), (1000, 11008, 4096, 0)]
 GEMM_O4_CASES = [(16, 1), (16, 0), (33, 0), (100, 0), (1000, 0)]      # flags 0 = the default dispatch (o4 never splits K)
 DECODE_LAYERS = 3
 

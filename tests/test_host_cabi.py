@@ -53,6 +53,17 @@ def test_kv_page_table_matches_reference_semantics():
         KvCacheInt4(pool, -1)
 
 
+def test_gemm_rejects_unknown_flag_bits_before_touching_the_device():
+    """A flag bit the library does not know (512 selected a GEMM kernel that has been removed) fails loudly instead of
+    quietly running another kernel.  The check comes before any device work, so dummy pointers suffice."""
+    from atom_b200 import _lib
+    l = _lib.lib()
+    p = [0x10000 + 0x100 * i for i in range(9)]          # 16-byte aligned, never dereferenced
+    rc = l.atom_gemm_i4_o16(*p, 16, 256, 512, 512, None)
+    assert rc == -1                                       # ATOM_E_INVALID
+    assert "flags" in l.atom_last_error().decode()
+
+
 def test_ops_reject_wrong_element_types_before_touching_the_device():
     """The C ABI takes raw pointers: the Python mirror refuses tensors whose element width cannot be what the kernel reads."""
     from atom_b200 import ops

@@ -30,7 +30,7 @@ def ulp(a, b):
 
 def diag():
     cases = [(16, 128, 256, 1), (16, 128, 512, 1), (16, 256, 4096, 1), (16, 256, 4096, 0), (7, 384, 1024, 32), (32, 256, 2048, 16),
-             (64, 128, 1024, 1), (16, 128, 256, 129), (128, 128, 512, 2)]
+             (64, 128, 1024, 1), (128, 128, 512, 2)]
     if len(sys.argv) > 2:
         cases = [tuple(int(x) for x in a.split(",")) for a in sys.argv[2:]]
     for (m, n, k, flags) in cases:
@@ -143,15 +143,10 @@ def gtiming(ms_list, n=4096, k=4096):
         ops_count = 2.0 * m * n * k
         rec = {"graph_time": [m, n, k], "rot_sets": nrot}
         variants = {"auto": 0, "nosplit": 1}
-        if m <= 64:
-            variants["legacy"] = 128
-            variants["legacy_nosplit"] = 129
-        elif m <= 128:
+        if 64 < m <= 128:
             variants["skinny"] = 4
         if m > 64:
-            variants["tall128"] = 1024        # 128 x 128 tiles
-            variants["wide256"] = 512         # 128 x 256 tiles, token operand in tensor memory
-            variants["legacy_tall"] = 256
+            variants["tall128"] = 2           # 128 x 128 tiles
         launches = nrot if m <= 512 else 6
         for name, flags in variants.items():
             us = graph_time(lambda i: ops.dense_layer_gemm_i4_fp16(*sets[i % nrot], flags=flags), nrot, launches=launches)
@@ -251,7 +246,7 @@ if __name__ == "__main__":
             nrot = max(3, int(300e6 // per_set) + 1)
             sets = [[T(x) for x in base] for _ in range(nrot)]
             rec = {"gshape": [m, n, k]}
-            for name, flags in {"auto": 0, "nosplit": 1, "split2": 16, "split4": 32, "split8": 64, "legacy_auto": 128}.items():
+            for name, flags in {"auto": 0, "nosplit": 1, "split2": 16, "split4": 32, "split8": 64}.items():
                 us = graph_time(lambda i: ops.dense_layer_gemm_i4_fp16(*sets[i % nrot], flags=flags), nrot, launches=nrot)
                 rec[name] = round(us, 2)
             print(json.dumps(rec), flush=True)

@@ -3,7 +3,7 @@
 # ncu is a bench value.  Outputs in gpurun_out/; summarise the .ncu-rep files HERE afterwards with tools/ncu_summary.py
 # and copy the summaries into profiles/.
 #   /usr/local/graft/bin/gpurun --timeout 1200 -- 'bash tools/gpu_prof.sh [steps...]'
-# steps (default: launches traffic gemm decode quant layer; extra: f16path)
+# steps (default: launches traffic gemm decode quant layer)
 set -u
 mkdir -p gpurun_out
 OUT=gpurun_out
@@ -22,8 +22,6 @@ for s in $STEPS; do case $s in
   gemm)     timeout 300 ncu $FULL -k regex:gemm_ -s 3 -c 1 -f -o $OUT/prof_gemm_m16_split python tools/prof_gemm.py 16 0 > /dev/null 2>&1
             timeout 300 ncu $FULL -k regex:gemm_ -s 3 -c 1 -f -o $OUT/prof_gemm_m16_nosplit python tools/prof_gemm.py 16 1 > /dev/null 2>&1
             timeout 300 ncu $FULL -k regex:gemm_ -s 3 -c 1 -f -o $OUT/prof_gemm_m4096_tall python tools/prof_gemm.py 4096 2 > /dev/null 2>&1 ;;
-  f16path)  # experimental FP16-path prefill kernel (flags 2|64)
-            timeout 300 ncu $FULL -k regex:gemm_ -s 3 -c 1 -f -o $OUT/prof_gemm_m4096_f16path python tools/prof_gemm.py 4096 66 > /dev/null 2>&1 ;;
   decode)   timeout 300 ncu $FULL -k regex:batch_decode -s 2 -c 1 -f -o $OUT/prof_decode python tools/layer_bench.py --copies 1 > /dev/null 2>&1 ;;
   quant)    timeout 300 ncu $FULL -k regex:rmsnorm -s 2 -c 1 -f -o $OUT/prof_rmsnorm python tools/layer_bench.py --copies 1 > /dev/null 2>&1 ;;
   layer)    # per-kernel times of one decode step of a Llama-7B layer
